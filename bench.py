@@ -2,6 +2,7 @@
 """Benchmark of the FlowMap optimisation hot path on B200 (contract: DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode scenes|pairs]
+                    [--dump-outputs DIR]
 
 One "step" = one full overfit iteration at BASELINE config 3 (150 x 360 x 640, synthetic):
 explicit-depth backbone, all-pixel Procrustes, softmin intrinsics (60-candidate sweep), flow
@@ -11,6 +12,9 @@ default losses/intrinsics and `+experiment=ablation_explicit_depth`.
 N > 1 (default --mode scenes, BASELINE config 5): one independent scene per GPU, no data-path
 collective.  --mode pairs (config 4 style): flow-loss-only run of ONE long video whose frame
 pairs are sharded across ranks, one all-reduce per step.  Prints ONE JSON line on rank 0.
+--dump-outputs DIR writes what the last timed step computed on rank 0 as DIR/<name>.npy (see
+dump_outputs); the inputs are seeded, so two builds can be compared output for output.
+The benchmark writes nothing into the source tree.
 """
 from __future__ import annotations
 
@@ -27,6 +31,7 @@ import torch
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the tree may be read-only; leave no __pycache__ in it
 
 F_, H_, W_ = 150, 360, 640  # BASELINE.json configs[2] ("Tanks&Temples-shape")
 START_STEP = 50             # tracking loss enabled (>= 50), softmin stage (< 1000)
@@ -69,6 +74,34 @@ def synthetic_track_arrays(f, n_points=1225, interval=5, radius=20, seed=0):
 def algorithmic_bytes(f, h, w):
     """SURVEY 8(d): 32 B per pair-pixel + 8 B per frame-pixel."""
     return h * w * (32 * (f - 1) + 8 * f)
+
+
+DUMP_SAMPLE = 1 << 21  # elements kept of each per-pixel array (4 arrays x 8 MB)
+
+
+def dump_outputs(out_dir, o, last):
+    """Write what the last step of `o` computed, as float32 .npy files under `out_dir`: the total
+    loss and relative poses it returned, the (fx, fy, cx, cy) it used, the focal-length gradient,
+    and of the per-pixel arrays (updated depth and weight logits, their gradients; 138 MB each at
+    the benchmark shape) the same fixed, seeded sample of elements in every run."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    loss, rt = last
+    grads = o.gradients()
+    arrays = {"loss": loss, "rt": rt, "intrinsics_k4": o.intrinsics_k4(), "g_focal": grads["focal"]}
+    per_pixel = {"depth": o.model.backbone.depth, "weight_logits": o.model.backbone.weights,
+                 "g_depth": grads["depth"], "g_weight_logits": grads["weights"]}
+    picks = {}
+    for name, t in per_pixel.items():
+        flat = t.detach().reshape(-1)
+        n = flat.numel()
+        if n not in picks:
+            g = torch.Generator().manual_seed(n)
+            picks[n] = torch.randperm(n, generator=g)[:DUMP_SAMPLE].sort().values.to(flat.device)
+        arrays[f"{name}_sample"] = flat[picks[n]]
+    for name, t in arrays.items():
+        np.save(out_dir / f"{name}.npy", t.detach().float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------ clocks
@@ -498,6 +531,8 @@ def run_gpu(args):
     pairs_mode = args.mode in ("pairs", "pairs-full")
     pairs_full = args.mode == "pairs-full"
 
+    # the step clock draws the seed of its softmin point sample from torch's generator
+    torch.manual_seed(rank)
     inputs = synthetic_inputs(F_, H_, W_, seed=rank)
     batch = Batch(torch.zeros(1, 1, 1, 1, 1, device=dev).expand(1, F_, 3, H_, W_),
                   torch.arange(F_, device=dev)[None], ["synthetic"], ["synthetic"])
@@ -585,6 +620,8 @@ def run_gpu(args):
     l0 = lib().fm_launch_count()
     ms, last = time_steps(o.training_step, args.steps)
     launches = lib().fm_launch_count() - l0
+    if args.dump_outputs and rank == 0:  # before the legs below run more steps on `o`
+        dump_outputs(args.dump_outputs, o, last)
     graph_replay = bool(getattr(o, "_graphs", None))
     if graph_replay:  # replayed graph nodes are not host launches: count the kernels they contain
         launches = launches_per_step * args.steps
@@ -861,8 +898,7 @@ def run_gpu(args):
 def run_reference(args):
     """The reference's own CPU implementation of the path: the UNMODIFIED reference modules staged
     under baseline/_ref (baseline/install_ref.py) on the full C3 workload; if they are missing
-    (a checkout that never ran build() next to /root/reference) the oracle port on a bounded
-    sample, labelled as such."""
+    (baseline/install_ref.py was not run) the oracle port on a bounded sample, labelled as such."""
     if int(os.environ.get("RANK", 0)) != 0:
         return
     if reference_available() and args.mode == "scenes":
@@ -900,7 +936,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--mode", default="scenes", choices=["scenes", "pairs", "pairs-full"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -11,9 +11,9 @@ The inputs are NOT stored: they are `bench.synthetic_inputs(f, h, w, seed)` and
 `bench.synthetic_track_arrays(f, seed=seed)` (torch's seeded CPU generator), which the GPU
 tests regenerate; the fixture keeps the reference's outputs in reduced form -- loss parts,
 all poses, the focal length, and for every full-size gradient / parameter tensor its per-frame
-L2 norms plus a strided subsample (every 61st element: 61 is prime to the row lengths, so the
-samples wander through all columns).  The Lightning shell is restated as in make_golden.py
-(model_wrapper_overfit.py:51-73, 104-105); the softmin point indices are injected by patching
+L2 norms plus a strided subsample (every STRIDES[case]-th element: multiples of 61, so that the
+samples wander through the columns, chosen to keep every fixture under 1 MB).  The Lightning
+shell is restated as in make_golden.py (model_wrapper_overfit.py:51-73, 104-105); the softmin point indices are injected by patching
 torch.randperm (SURVEY A.8 item 1): the first `softmin_points` entries of
 torch.randperm(h * w, generator=manual_seed(3)).
 """
@@ -31,7 +31,7 @@ REF = "/root/reference"
 OUT = Path(__file__).resolve().parent
 ROOT = OUT.parent.parent
 sys.path.insert(0, str(ROOT))
-STRIDE = 61
+STRIDES = {"c2": 122, "c3": 732, "c4slice": 488}
 START_STEP = 50  # bench.START_STEP: tracking loss on (>= 50), softmin stage (< 1000)
 
 
@@ -82,8 +82,7 @@ def main():
     from flowmap.tracking.track_predictor import Tracks
 
     global STRIDE
-    if which in ("c3", "c4slice"):
-        STRIDE = 244  # keeps the fixtures at ~2 MB
+    STRIDE = STRIDES[which]
     seed = 0
     inp = {k: v.to(dtype) for k, v in inp32.items()}
     if intr == "softmin":
